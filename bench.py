@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the north-star path: tumbling fold_window count-by-key (config C1).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (SURVEY.md section 8d, BASELINE.json configs[1]): rows (u64 key, u64 val),
 key_i = splitmix64(0x5EED ^ i) mod 10^6, val_i = ts_i = i us after 2022-01-01,
@@ -18,6 +18,13 @@ host cores, bounded sample.
 
 `--impl reference` times that CPU restatement alone (the reference's Rust
 engine cannot be built here: no cargo, un-vendored timely -- DESIGN.md).
+
+`--dump-outputs DIR` writes, after the timed steps, the rows the timed job hands
+its caller: `bw_advance` after the last timed step (every window the K steps
+closed) and `bw_eof` (the windows still open), one float64 `DIR/<name>.npy` per
+non-empty column (the C1 stream has no late rows, so no late columns).  The
+inputs depend only on the arguments, so two builds given the same arguments can
+be compared file by file.
 """
 
 import argparse
@@ -37,6 +44,7 @@ N_KEYS = 1_000_000
 WINDOW_US = 60_000_000
 BATCH_ROWS = 1 << 24
 BYTES_PER_EVENT = 16  # SURVEY.md 8(d): one read of the (u64, u64) record
+DUMP_BYTES = 60 << 20  # --dump-outputs writes at most this much: a seeded sample of each longer column
 
 
 def peaks():
@@ -267,15 +275,15 @@ def run_gpu(args):
         fold.ingest_device(dk[K + s], dv[K + s], None, B)
     fold.advance()
     fold.close()
-    # The K-step job takes tens of milliseconds: it is repeated (a fresh fold each time, created outside the timed
-    # region) until >= min_timed_s of timed device work has accumulated, so that the clock / throttle sampler sees the
-    # GPU under load; ms_per_step is the MEDIAN repetition (every repetition times exactly K steps).
+    # The timed region is exactly K steps on a fresh fold (created outside it).  --min-timed-s > 0 repeats that K-step job
+    # (a fresh fold each time) until that much timed device work has accumulated, so that the clock / throttle sampler
+    # sees the GPU under load; ms_per_step is then the MEDIAN repetition.
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     rep_ms, reps_total_ms = [], 0.0
     st0 = st1 = None
-    checks = None
+    checks = emitted = None
     while True:
         fold = make_fold()
         st0 = fold.stats()
@@ -295,10 +303,13 @@ def run_gpu(args):
             em = fold.advance()
             em_eof = fold.eof()
             checks = check_counts(em, em_eof, K, B, world, dist, local, args.ts_stride, args.late_frac)
+            emitted = (em, em_eof)
         fold.close()
         if not more:
             break
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"advance": emitted[0], "eof": emitted[1]})
     rep_ms.sort()
     ms = rep_ms[len(rep_ms) // 2]
     total_counts, per_window_ok = checks
@@ -384,6 +395,24 @@ def run_gpu(args):
         dist.destroy_process_group()
     if rank == 0:
         print(json.dumps(out))
+
+
+def dump_outputs(out_dir, streams):
+    """Every non-empty column of every `Emitted` as float64 `out_dir/<stream>_<column>.npy` (the bench's keys, window ids,
+    counts and epochs are far below 2^53, so the values are exact).  A column longer than its share of DUMP_BYTES is replaced by the
+    rows at a seeded, sorted sample of positions: the same positions for the same row count, so emission order still counts."""
+    import dataclasses
+
+    import numpy as np
+
+    cols = {f"{name}_{f.name}": getattr(em, f.name) for name, em in streams.items() for f in dataclasses.fields(em)}
+    cols = {name: a for name, a in cols.items() if len(a)}
+    cap = DUMP_BYTES // (8 * len(cols))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in cols.items():
+        if len(a) > cap:
+            a = a[np.sort(np.random.default_rng(0x5EED).choice(len(a), cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 def run_e2e(ctx, make_fold, K, B, rank, world, dist, local):
@@ -492,7 +521,6 @@ def run_reference(args):
     orcs = [coracle.COracle("count", WINDOW_US, align_us=ALIGN_US) for _ in range(T)]
     arr = (C.c_void_p * T)(*[o.h for o in orcs])
     K, W = args.steps, args.warmup
-    K = min(K, 16)  # keeps the whole run within minutes
     times = []
     for s in range(W + K):
         keys, ts, _ = coracle.gen_c1(s * rows, rows, N_KEYS, ALIGN_US)
@@ -644,25 +672,29 @@ def main():
         os.environ["NCCL_DEBUG"] = "WARN"
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=60)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 60 for c1, 8 for c2 | c3 | c4)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--batch-rows", type=int, default=BATCH_ROWS)
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"])
     ap.add_argument("--n-keys", type=int, default=N_KEYS, help="diagnostic: key cardinality (the metric is quoted at the default)")
     ap.add_argument("--ts-stride", type=int, default=1, help="diagnostic: event time advances this many us per row")
-    ap.add_argument("--min-timed-s", type=float, default=1.0, help="repeat the K-step job until this much timed device work")
+    ap.add_argument("--min-timed-s", type=float, default=0.0,
+                    help="repeat the K-step job (a fresh fold each time) until this much timed device work; ms_per_step is the median")
     ap.add_argument("--max-repeats", type=int, default=200)
     ap.add_argument("--late-frac", type=float, default=0.0, help="diagnostic: this fraction of the rows arrives 120 s late (exact path)")
     ap.add_argument("--config", default="c1", help="c1 (the headline metric, default); c2 | c3 | c4: secondary lines for BASELINE.json configs[2..4]")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the rows the timed job emits to DIR/<name>.npy (c1 on the GPU only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config != "c1"):
+        ap.error("--dump-outputs needs the c1 GPU path")
+    if args.steps is None:
+        args.steps = 60 if args.config == "c1" else 8
     if args.impl == "reference":
         run_reference(args)
     elif args.config != "c1":
-        if args.steps == 60:
-            args.steps = 8
         run_config(args)
     else:
         run_gpu(args)

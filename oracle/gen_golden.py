@@ -1,8 +1,8 @@
 """Generate ``tests/golden/*.json`` from the UNMODIFIED reference Python logic.
 
-TEST INFRASTRUCTURE ONLY.  Run in the build container (needs /root/reference):
+TEST INFRASTRUCTURE ONLY.  Needs a source checkout of the reference (bytewax v0.21.1):
 
-    python oracle/gen_golden.py
+    BYTEWAX_SRC=<checkout> python oracle/gen_golden.py
 
 For every case it builds a real reference flow (``win.count_window`` /
 ``win.reduce_window`` / ``win.max_window`` / ``win.min_window`` /
@@ -16,7 +16,9 @@ The cases named ``ref_*`` restate inputs of the reference's own tests and are
 additionally asserted against the expected lists written in those tests.
 """
 
+import gzip
 import json
+import math
 import os
 import random
 import sys
@@ -26,6 +28,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 
 from oracle import refstub  # noqa: E402
+from oracle.streams import ALIGN_US, gen_random, random_case, spec_, sweep_case  # noqa: E402
 
 win = refstub.load()
 import bytewax.operators as op  # noqa: E402  (the reference's)
@@ -33,7 +36,6 @@ from bytewax.dataflow import Dataflow  # noqa: E402
 from bytewax.testing import TestingSource  # noqa: E402
 
 EPOCH = datetime(1970, 1, 1, tzinfo=timezone.utc)
-ALIGN_US = 1_640_995_200_000_000  # 2022-01-01T00:00:00Z
 NOW = datetime(2030, 1, 1, tzinfo=timezone.utc)
 
 
@@ -150,30 +152,6 @@ def run_reference(spec, batches):
         rows.extend(conv(ks, list(events)))
     acts.append(rows)
     return acts
-
-
-def spec_(reduction="count", length_us=10_000_000, offset_us=None, wait_us=0, ordered=False, align_us=ALIGN_US):
-    return dict(
-        reduction=reduction, length_us=length_us, offset_us=offset_us, wait_us=wait_us, ordered=ordered, align_us=align_us
-    )
-
-
-def gen_random(seed, n, n_keys, span_us, jitter_us, batch_sizes, fval=False, start_us=ALIGN_US, key_base=0):
-    rnd = random.Random(seed)
-    keys, ts, vals = [], [], []
-    for i in range(n):
-        base = start_us + (i * span_us) // n
-        t = base + rnd.randint(-jitter_us, jitter_us) if jitter_us else base
-        keys.append(key_base + rnd.randrange(n_keys))
-        ts.append(t)
-        vals.append(round(rnd.uniform(-100, 100), 3) if fval else rnd.randint(-1000, 1000))
-    batches, i, b = [], 0, 0
-    while i < n:
-        sz = batch_sizes[b % len(batch_sizes)]
-        batches.append([keys[i : i + sz], ts[i : i + sz], vals[i : i + sz]])
-        i += sz
-        b += 1
-    return batches
 
 
 def main():
@@ -456,7 +434,7 @@ def main_timed():
 
 def main_keyed():
     """Goldens for config C2 (the reference example's own mapper) and C4 (the reference's `_JoinLogic`)."""
-    src = open("/root/reference/examples/anomaly_detector.py").read()
+    src = open(os.path.join(refstub.REFERENCE_ROOT, "examples", "anomaly_detector.py")).read()
     ns = {}
     start, end = src.index("@dataclass\nclass DetectorState"), src.index("labeled_metrics =")
     exec("from dataclasses import dataclass, field\nfrom typing import List, Optional\n" + src[start:end], ns)  # examples/anomaly_detector.py:16-48
@@ -497,7 +475,133 @@ def main_keyed():
     print("wrote", path, os.path.getsize(path), "bytes")
 
 
+def main_sweep():
+    """tests/golden/reference_sweep_cases.json.gz: the reference's rows per activation for the seeded specs and streams of
+    `oracle.streams.random_case` (seeds 30..35) and `sweep_case` (seeds 100..147); the inputs are regenerated from the seeds."""
+    out = {"random": {}, "sweep": {}}
+    for name, make, seeds in (("random", random_case, range(30, 36)), ("sweep", sweep_case, range(100, 148))):
+        for seed in seeds:
+            spec, batches = make(seed)
+            out[name][str(seed)] = dict(spec=spec, acts=run_reference(spec, batches))
+    path = os.path.join(os.path.dirname(HERE), "tests", "golden", "reference_sweep_cases.json.gz")
+    with gzip.GzipFile(path, "wb", mtime=0) as f:
+        f.write(json.dumps(out, separators=(",", ":")).encode())
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+
+SNAPSHOT_PARAMS = [("count", 10, None, 0), ("sum", 10, None, 3), ("sum", 10, 5, 2), ("max", 12, 4, 1)]
+I64_MIN = -(1 << 63)
+
+
+def _device_columns(accepted, opened_by_key, max_ts, red, length, offset, closed_upto):
+    """What the device table holds at the cut: per key the live panes (those under a still-open window) with the fold of the
+    accepted items in them, the first arrival index per pane, the key's running maximum and its `closed_upto`."""
+    g = math.gcd(length, offset)
+    a, b = offset // g, length // g
+    cols = {n: [] for n in ("key", "pane_id", "acc", "count", "open_seq", "max_ts_us", "closed_upto")}
+    fold = {"count": lambda x, v: x + 1, "sum": lambda x, v: x + v, "min": min, "max": max}[red]
+    for k, opened in opened_by_key.items():
+        panes = {}
+        for seq, ts, v in accepted[k]:
+            q = (ts - ALIGN_US) // g
+            w_lo, w_hi = -((-(q - b + 1)) // a), q // a
+            if not any(w in opened for w in range(w_lo, w_hi + 1)):
+                continue  # every window of this pane has closed: the pane is gone
+            cur = panes.get(q)
+            if cur is None:
+                panes[q] = [(1 if red == "count" else v), seq]
+            else:
+                cur[0] = fold(cur[0], v)
+        for q, (acc, seq) in sorted(panes.items()):
+            cols["key"].append(k)
+            cols["pane_id"].append(q)
+            cols["acc"].append(acc & 0xFFFFFFFFFFFFFFFF)
+            cols["count"].append(0)
+            cols["open_seq"].append(seq)
+            cols["max_ts_us"].append(max_ts[k])
+            cols["closed_upto"].append(closed_upto.get(k, I64_MIN))
+    return cols
+
+
+def main_snapshots():
+    """tests/golden/snapshot_resume_cases.json: a seeded stream folded by the reference's `_WindowLogic` objects up to a cut;
+    the state at the cut written the way the device dumps it (one row per live (key, pane): what `bw_snapshot_take`
+    returns), the reference's own `snapshot()` of every key at the cut, and the rows the uninterrupted logics emit after it."""
+    S = 1_000_000
+    cases = []
+    for ci, (red, length, offset, wait) in enumerate(SNAPSHOT_PARAMS):
+        spec = spec_(red, length * S, offset * S if offset else None, wait * S, False)
+        off = spec["offset_us"] or spec["length_us"]
+        rnd = random.Random(7000 + ci)
+        batches, t = [], ALIGN_US
+        for _ in range(12):
+            n = rnd.randint(20, 60)
+            keys = [rnd.randint(1, 9) for _ in range(n)]
+            ts = [t + rnd.randint(0, 6 * S) - (rnd.randint(0, 8 * S) if rnd.random() < 0.2 else 0) for _ in range(n)]
+            t += 5 * S
+            batches.append([keys, ts, [rnd.randint(-20, 20) for _ in range(n)]])
+        cut = 6
+        builder, unwrap = build_logic_builder(spec)
+
+        def drive(logics, chunk, seq0, accepted=None, max_ts=None):
+            rows = []
+            for bi, (keys, ts, vals) in enumerate(chunk):
+                grouped = {}
+                for i, (k, tt, v) in enumerate(zip(keys, ts, vals)):
+                    grouped.setdefault(str(k), []).append((str(k), v, tt, (seq0 + bi) << 32 | i))
+                for ks in sorted(grouped):
+                    logic = logics.get(ks)
+                    if logic is None:
+                        logic = logics[ks] = builder(None)
+                    events, done = logic.on_batch([(k, v, tt) for k, v, tt, _s in grouped[ks]])
+                    events = list(events)
+                    late_vals = [p[1] for _w, tag, p in events if tag == "L"]
+                    for k, v, tt, sq in grouped[ks]:
+                        if accepted is not None:
+                            if late_vals and v in late_vals and any(p[2] == tt for _w, tag, p in events if tag == "L"):
+                                continue
+                            accepted.setdefault(int(ks), []).append((sq, tt, v))
+                            max_ts[int(ks)] = max(max_ts.get(int(ks), I64_MIN), tt)
+                    rows.extend([ks, w, tag, (unwrap(p) if tag == "E" else None)] for w, tag, p in events if tag != "M")
+                    if done:
+                        del logics[ks]
+                        if accepted is not None:  # the key's state is gone with its logic (discard resets the watermark)
+                            accepted.pop(int(ks), None)
+                            max_ts.pop(int(ks), None)
+            return rows
+
+        # uninterrupted
+        ref_logics = {}
+        drive(ref_logics, batches[:cut], 0)
+        want = drive(ref_logics, batches[cut:], cut)
+        want_eof = [[ks, w, tag, unwrap(p) if tag == "E" else None] for ks in sorted(ref_logics)
+                    for w, tag, p in ref_logics[ks].on_eof()[0] if tag != "M"]
+        # up to the cut, remembering what the table would hold
+        logics, accepted, max_ts = {}, {}, {}
+        drive(logics, batches[:cut], 0, accepted, max_ts)
+        opened_by_key = {int(ks): dict(lg.windower.state.opened) for ks, lg in logics.items()}
+        # sliding windows: every id below the oldest open one that covers a live pane has been emitted
+        closed_upto = {k: (min(o) - 1 if (offset and o) else I64_MIN) for k, o in opened_by_key.items()}
+        cols = _device_columns(accepted, opened_by_key, max_ts, red, spec["length_us"], off, closed_upto)
+        snaps = {}
+        for ks, lg in logics.items():
+            real = lg.snapshot()
+            snaps[ks] = dict(
+                opened=[[w, us(m.open_time), us(m.close_time)] for w, m in real.windower_state.opened.items()],
+                logic_states=[[w, unwrap(v) if red != "count" else v] for w, v in real.logic_states.items()],
+                clock_delta_us=us(real.clock_state.watermark_base) - us(real.clock_state.system_time_of_max_event),
+            )
+        cases.append(dict(params=[red, length, offset, wait], spec=spec, now_us=us(NOW), cut=cut, batches=batches,
+                          columns=cols, snapshots=snaps, want=want, want_eof=want_eof))
+    path = os.path.join(os.path.dirname(HERE), "tests", "golden", "snapshot_resume_cases.json")
+    with open(path, "w") as f:
+        json.dump(cases, f, separators=(",", ":"))
+    print("wrote", path, os.path.getsize(path), "bytes,", len(cases), "cases")
+
+
 if __name__ == "__main__":
     main()
     main_keyed()
     main_timed()
+    main_sweep()
+    main_snapshots()

@@ -1,8 +1,8 @@
 """Import the reference's *Python half* in place.  TEST INFRASTRUCTURE ONLY.
 
-Works only where ``/root/reference`` exists (the build container; never the
-GPU box).  Used by ``oracle/gen_golden.py`` to produce ``tests/golden/*.json``
-and by ``tests/test_oracle_vs_reference.py`` (skipped when the tree is absent).
+Works only where a source checkout of the reference (bytewax v0.21.1) is given
+in ``$BYTEWAX_SRC``.  Used by ``oracle/gen_golden.py`` to produce
+``tests/golden/*``.
 
 The reference's engine is Rust (``bytewax._bytewax``, src/lib.rs:24-32) and
 cannot be built here (no cargo, un-vendored timely; SURVEY.md section 8c).  Its
@@ -14,17 +14,18 @@ import os
 import sys
 import types
 
-REFERENCE_PYSRC = "/root/reference/pysrc"
+REFERENCE_ROOT = os.environ.get("BYTEWAX_SRC", "")
+REFERENCE_PYSRC = os.path.join(REFERENCE_ROOT, "pysrc") if REFERENCE_ROOT else ""
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_PYSRC, "bytewax"))
+    return bool(REFERENCE_PYSRC) and os.path.isdir(os.path.join(REFERENCE_PYSRC, "bytewax"))
 
 
 def load():
     """Return the reference's ``bytewax.operators.windowing`` module."""
     if not available():
-        raise RuntimeError("reference tree not present")
+        raise RuntimeError("reference checkout not found: set BYTEWAX_SRC to a bytewax v0.21.1 source tree")
     if "bytewax" in sys.modules and not getattr(sys.modules["bytewax"], "__file__", "").startswith(
         REFERENCE_PYSRC
     ):

@@ -2,12 +2,12 @@
 reference's own, unmodified window logic (oracle/gen_golden.py) and against the
 expected lists of the reference's tests (cases named ref_*)."""
 
+import gzip
 import json
 import os
 
-import pytest
-
 from oracle import pyoracle as po
+from oracle import streams
 
 
 def _load(golden_dir, name):
@@ -113,70 +113,56 @@ def test_clock_reference_test_values():
     assert c2.on_item(8 * S)[1] == 5 * S  # does not reverse
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/pysrc"), reason="reference tree absent")
-def test_oracle_vs_live_reference_random():
-    """Extra seeds straight against the live reference (build container only)."""
-    import subprocess
-    import sys
-
-    code = (
-        "import sys, json; sys.path.insert(0, %r); sys.argv=['x'];"
-        "import oracle.gen_golden as g; from oracle import pyoracle as po;"
-        "S=10**6\n"
-        "for seed in range(30, 36):\n"
-        "    spec=g.spec_(['count','sum','min','max'][seed%%4], 10*S, [None,5*S,3*S][seed%%3], wait_us=(seed%%4)*S, ordered=bool(seed%%2) and (seed%%4)<2)\n"
-        "    b=g.gen_random(seed, 400, 7, 50*S, 4*S, [17, 60])\n"
-        "    want=g.run_reference(spec,b)\n"
-        "    got=po.run_fold(po.FoldSpec(spec['reduction'],spec['length_us'],spec['offset_us'],spec['align_us'],spec['wait_us'],spec['ordered']), b)\n"
-        "    got=[[[k,w,t,list(p) if isinstance(p,tuple) else p] for k,w,t,p in a] for a in got]\n"
-        "    assert got==want, seed\n"
-        "print('ok')\n"
-    ) % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
+def _reference_sweep(golden_dir):
+    with gzip.open(os.path.join(golden_dir, "reference_sweep_cases.json.gz")) as f:
+        return json.load(f)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/pysrc"), reason="reference tree absent")
-def test_oracles_vs_live_reference_sweep():
-    """Wider differential sweep in the build container: 48 seeded specs (all five reductions, tumbling / sliding with divisible and
-    indivisible offsets, waits from 0 to beyond the data span, ordered and unordered, timestamps on both sides of align_to, bursts of
-    late items) through the reference's unmodified `_WindowLogic`, the Python oracle and the C oracle: identical per activation."""
-    import subprocess
-    import sys
+def _py_rows(spec, batches):
+    fs = po.FoldSpec(spec["reduction"], spec["length_us"], spec["offset_us"], spec["align_us"], spec["wait_us"], spec["ordered"])
+    return [[[k, w, t, list(p) if isinstance(p, tuple) else p] for k, w, t, p in a] for a in po.run_fold(fs, batches)]
 
-    code = (
-        "import sys, json; sys.path.insert(0, %r); sys.argv=['x'];"
-        "import numpy as np; import oracle.gen_golden as g; from oracle import pyoracle as po, coracle;"
-        "S=10**6\n"
-        "n=0\n"
-        "for seed in range(100, 148):\n"
-        "    red=['count','sum','min','max','mean'][seed%%5]\n"
-        "    length=[10*S, 7*S, 60*S, 1*S][seed%%4]\n"
-        "    offset=[None, length//2 or None, 3*S if 3*S<length else None][seed%%3]\n"
-        "    wait=[0, S, 4*S, 500*S][(seed//3)%%4]\n"
-        "    ordered=bool((seed//5)%%2) and red in ('count','sum','mean')  # max/min_window are always unordered (windowing.py:2189, 2236)\n"
-        "    spec=g.spec_(red, length, offset, wait_us=wait, ordered=ordered)\n"
-        "    b=g.gen_random(seed, 300, 5, 40*S, [0, 2*S, 9*S][seed%%3], [11, 50, 7], start_us=g.ALIGN_US-15*S)\n"
-        "    want=g.run_reference(spec,b)\n"
-        "    fs=po.FoldSpec(spec['reduction'],spec['length_us'],spec['offset_us'],spec['align_us'],spec['wait_us'],spec['ordered'])\n"
-        "    got=po.run_fold(fs, b)\n"
-        "    got=[[[k,w,t,list(p) if isinstance(p,tuple) else p] for k,w,t,p in a] for a in got]\n"
-        "    assert got==want, ('py', seed)\n"
-        "    if red!='mean':\n"
-        "        orc=coracle.COracle(red, length, offset, g.ALIGN_US, wait, ordered)\n"
-        "        for keys,ts,vals in b: orc.on_batch(np.array(keys,dtype=np.uint64), np.array(ts,dtype=np.int64), np.array(vals,dtype=np.int64))\n"
-        "        orc.on_eof()\n"
-        "        ck,cw,ca,_,cact=orc.closed(); lk,lw,lv,_,lact=orc.late()\n"
-        "        wantE=[(a,k,w,p) for a,act in enumerate(want) for k,w,t,p in act if t=='E']\n"
-        "        wantL=[(a,k,w,p) for a,act in enumerate(want) for k,w,t,p in act if t=='L']\n"
-        "        assert list(zip(cact.tolist(),ck.tolist(),cw.tolist(),ca.tolist()))==wantE, ('c closed', seed)\n"
-        "        assert list(zip(lact.tolist(),lk.tolist(),lw.tolist(),lv.tolist()))==wantL, ('c late', seed)\n"
-        "        orc.close()\n"
-        "    n+=1\n"
-        "print('ok', n)\n"
-    ) % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "ok 48" in r.stdout, (r.stdout[-500:], r.stderr[-3000:])
+
+def test_oracle_vs_live_reference_random(golden_dir):
+    """Extra seeds against the rows the reference's unmodified `_WindowLogic` produced for them (oracle/gen_golden.py)."""
+    cases = _reference_sweep(golden_dir)["random"]
+    assert sorted(map(int, cases)) == list(range(30, 36))
+    for seed, case in cases.items():
+        spec, batches = streams.random_case(int(seed))
+        assert spec == case["spec"], seed
+        assert _py_rows(spec, batches) == case["acts"], seed
+
+
+def test_oracles_vs_live_reference_sweep(golden_dir):
+    """Wider differential sweep: 48 seeded specs (all five reductions, tumbling / sliding with divisible and indivisible
+    offsets, waits from 0 to beyond the data span, ordered and unordered, timestamps on both sides of align_to, bursts of
+    late items); the Python oracle and the C oracle against the rows the reference's unmodified `_WindowLogic` produced for
+    them (oracle/gen_golden.py): identical per activation."""
+    import numpy as np
+
+    from oracle import coracle
+
+    cases = _reference_sweep(golden_dir)["sweep"]
+    assert sorted(map(int, cases)) == list(range(100, 148))
+    for seed, case in cases.items():
+        spec, b = streams.sweep_case(int(seed))
+        assert spec == case["spec"], seed
+        want = case["acts"]
+        assert _py_rows(spec, b) == want, ("py", seed)
+        red = spec["reduction"]
+        if red == "mean":
+            continue
+        orc = coracle.COracle(red, spec["length_us"], spec["offset_us"], spec["align_us"], spec["wait_us"], spec["ordered"])
+        for keys, ts, vals in b:
+            orc.on_batch(np.array(keys, dtype=np.uint64), np.array(ts, dtype=np.int64), np.array(vals, dtype=np.int64))
+        orc.on_eof()
+        ck, cw, ca, _, cact = orc.closed()
+        lk, lw, lv, _, lact = orc.late()
+        want_e = [(a, k, w, p) for a, act in enumerate(want) for k, w, t, p in act if t == "E"]
+        want_l = [(a, k, w, p) for a, act in enumerate(want) for k, w, t, p in act if t == "L"]
+        assert list(zip(cact.tolist(), ck.tolist(), cw.tolist(), ca.tolist())) == want_e, ("c closed", seed)
+        assert list(zip(lact.tolist(), lk.tolist(), lw.tolist(), lv.tolist())) == want_l, ("c late", seed)
+        orc.close()
 
 
 def test_keyed_oracles_match_reference_goldens(golden_dir):

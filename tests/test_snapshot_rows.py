@@ -1,150 +1,98 @@
 """`bytewax_b200.snapshot_rows`: the columnar device snapshot turned into the reference's per-key `_WindowSnapshot` objects.
 
-The check runs the reference's OWN classes (imported from /root/reference through oracle/refstub.py, as oracle/gen_golden.py does;
-skipped where the reference is absent): a stream is folded by the real `_WindowLogic` objects up to a cut, the state at the cut is
-written the way the device dumps it (one row per live (key, pane): what `bw_snapshot_take` returns), converted, handed to the
-real builder as `resume_state`, and the resumed logics must emit exactly what the uninterrupted ones do."""
-import math
+`tests/golden/snapshot_resume_cases.json` (oracle/gen_golden.py) holds, per case, a seeded stream folded by the reference's OWN
+`_WindowLogic` objects up to a cut: the state at the cut written the way the device dumps it (one row per live (key, pane): what
+`bw_snapshot_take` returns), the reference's own `snapshot()` of every key there, and the rows the uninterrupted logics emit
+after the cut.  The columns are converted, must equal the reference's snapshots, are handed to the builder of `count_window` as
+`resume_state`, and the resumed logics must emit exactly what the uninterrupted reference logics did."""
+import json
 import os
 import pickle
-import random
-import sys
+from datetime import datetime, timedelta, timezone
 
 import numpy as np
 import pytest
 
+from oracle.refstub import find_stateful_batch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/pysrc"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference checkout (this container only)")
 
-ALIGN = 1_640_995_200_000_000
+EPOCH = datetime(1970, 1, 1, tzinfo=timezone.utc)
 S = 1_000_000
-I64_MIN = -(1 << 63)
 
 
-_GEN = []
+def _us(d):
+    delta = d - EPOCH
+    return (delta.days * 86400 + delta.seconds) * 1_000_000 + delta.microseconds
 
 
-def _gen():
-    if _GEN:
-        return _GEN[0]
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import importlib.util
-
-    spec = importlib.util.spec_from_file_location("gen_golden_for_rows", os.path.join(ROOT, "oracle", "gen_golden.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    _GEN.append(mod)
-    return mod
+def _cases():
+    with open(os.path.join(ROOT, "tests", "golden", "snapshot_resume_cases.json")) as f:
+        return {tuple(c["params"]): c for c in json.load(f)}
 
 
-def _device_columns(accepted, opened_by_key, max_ts, red, length, offset, closed_upto):
-    """What the table holds at the cut: per key the live panes (those under a still-open window) with the fold of the
-    accepted items in them, the first arrival index per pane, the key's running maximum and its `closed_upto`."""
-    g = math.gcd(length, offset)
-    a, b = offset // g, length // g
-    cols = {n: [] for n in ("key", "pane_id", "acc", "count", "open_seq", "max_ts_us", "closed_upto")}
-    fold = {"count": lambda x, v: x + 1, "sum": lambda x, v: x + v, "min": min, "max": max}[red]
-    for k, opened in opened_by_key.items():
-        panes = {}
-        for seq, ts, v in accepted[k]:
-            q = (ts - ALIGN) // g
-            w_lo, w_hi = -((-(q - b + 1)) // a), q // a
-            if not any(w in opened for w in range(w_lo, w_hi + 1)):
-                continue  # every window of this pane has closed: the pane is gone
-            cur = panes.get(q)
-            if cur is None:
-                panes[q] = [(1 if red == "count" else v), seq]
-            else:
-                cur[0] = fold(cur[0], v)
-        for q, (acc, seq) in sorted(panes.items()):
-            cols["key"].append(k)
-            cols["pane_id"].append(q)
-            cols["acc"].append(acc & 0xFFFFFFFFFFFFFFFF)
-            cols["count"].append(0)
-            cols["open_seq"].append(seq)
-            cols["max_ts_us"].append(max_ts[k])
-            cols["closed_upto"].append(closed_upto.get(k, I64_MIN))
-    dt = dict(key=np.uint64, pane_id=np.int64, acc=np.uint64, count=np.uint64, open_seq=np.uint64, max_ts_us=np.int64, closed_upto=np.int64)
-    return {n: np.array(v, dtype=dt[n]) for n, v in cols.items()}
+def _count_builder(spec, now_us):
+    """The `stateful_batch` builder of this package's `count_window` for the spec (items are `(key_str, value, ts_us)`)."""
+    import bytewax_b200.operators as op
+    from bytewax_b200.dataflow import Dataflow
+    from bytewax_b200.operators import windowing as win
+    from bytewax_b200.testing import TestingSource
+
+    dt = lambda us: EPOCH + timedelta(microseconds=us)  # noqa: E731
+    clock = win.EventClock(lambda x: dt(x[2]), wait_for_system_duration=timedelta(microseconds=spec["wait_us"]),
+                           now_getter=lambda: dt(now_us))
+    windower = win.SlidingWindower(length=timedelta(microseconds=spec["length_us"]),
+                                   offset=timedelta(microseconds=spec["offset_us"] or spec["length_us"]), align_to=dt(spec["align_us"]))
+    flow = Dataflow("g")
+    win.count_window("w", op.input("in", flow, TestingSource([])), clock, windower, lambda x: x[0])
+    return find_stateful_batch(flow).builder
+
+
+def _drive(logics, builder, chunk):
+    rows = []
+    for keys, ts, vals in chunk:
+        grouped = {}
+        for k, tt, v in zip(keys, ts, vals):
+            grouped.setdefault(str(k), []).append((str(k), v, tt))
+        for ks in sorted(grouped):
+            logic = logics.get(ks)
+            if logic is None:
+                logic = logics[ks] = builder(None)
+            events, done = logic.on_batch(grouped[ks])
+            rows.extend([ks, w, tag, (p if tag == "E" else None)] for w, tag, p in events if tag != "M")
+            if done:
+                del logics[ks]
+    return rows
 
 
 @pytest.mark.parametrize("red,length,offset,wait", [("count", 10, None, 0), ("sum", 10, None, 3), ("sum", 10, 5, 2), ("max", 12, 4, 1)])
 def test_resume_on_the_reference_logic(red, length, offset, wait):
-    gg = _gen()
     from bytewax_b200 import snapshot_rows
+    from bytewax_b200.operators import windowing as win
 
-    win = gg.win
-    spec = gg.spec_(red, length * S, offset * S if offset else None, wait * S, False)
+    case = _cases()[(red, length, offset, wait)]
+    spec, now_us = case["spec"], case["now_us"]
     off = spec["offset_us"] or spec["length_us"]
-    rnd = random.Random(hash((red, length)) & 0xFFFF)
-    batches, t = [], ALIGN
-    for _ in range(12):
-        n = rnd.randint(20, 60)
-        keys = [rnd.randint(1, 9) for _ in range(n)]
-        ts = [t + rnd.randint(0, 6 * S) - (rnd.randint(0, 8 * S) if rnd.random() < 0.2 else 0) for _ in range(n)]
-        t += 5 * S
-        batches.append((keys, ts, [rnd.randint(-20, 20) for _ in range(n)]))
-    cut = 6
-
-    def drive(logics, builder, chunk, unwrap, seq0, accepted=None, max_ts=None):
-        rows = []
-        for bi, (keys, ts, vals) in enumerate(chunk):
-            grouped = {}
-            for i, (k, tt, v) in enumerate(zip(keys, ts, vals)):
-                grouped.setdefault(str(k), []).append((str(k), v, tt, (seq0 + bi) << 32 | i))
-            for ks in sorted(grouped):
-                logic = logics.get(ks)
-                if logic is None:
-                    logic = logics[ks] = builder(None)
-                events, done = logic.on_batch([(k, v, tt) for k, v, tt, _s in grouped[ks]])
-                events = list(events)
-                late_vals = [p[1] for _w, tag, p in events if tag == "L"]
-                for k, v, tt, sq in grouped[ks]:
-                    if accepted is not None:
-                        if late_vals and v in late_vals and any(p[2] == tt for _w, tag, p in events if tag == "L"):
-                            continue
-                        accepted.setdefault(int(ks), []).append((sq, tt, v))
-                        max_ts[int(ks)] = max(max_ts.get(int(ks), I64_MIN), tt)
-                rows.extend((ks, w, tag, (unwrap(p) if tag == "E" else None)) for w, tag, p in events if tag != "M")
-                if done:
-                    del logics[ks]
-                    if accepted is not None:  # the key's state is gone with its logic (discard resets the watermark)
-                        accepted.pop(int(ks), None)
-                        max_ts.pop(int(ks), None)
-        return rows
-
-    builder, unwrap = gg.build_logic_builder(spec)
-    # uninterrupted
-    ref_logics = {}
-    drive(ref_logics, builder, batches[:cut], unwrap, 0)
-    want = drive(ref_logics, builder, batches[cut:], unwrap, cut)
-    want_eof = [(ks, w, tag, unwrap(p) if tag == "E" else None) for ks in sorted(ref_logics) for w, tag, p in ref_logics[ks].on_eof()[0] if tag != "M"]
-    # up to the cut, remembering what the table would hold
-    logics, accepted, max_ts = {}, {}, {}
-    drive(logics, builder, batches[:cut], unwrap, 0, accepted, max_ts)
-    opened_by_key = {int(ks): dict(lg.windower.state.opened) for ks, lg in logics.items()}
-    closed_upto = {}
-    for k, opened in opened_by_key.items():
-        # sliding windows: every id below the oldest open one that covers a live pane has been emitted
-        closed_upto[k] = min(opened) - 1 if (offset and opened) else I64_MIN
-    cols = _device_columns(accepted, opened_by_key, max_ts, red, spec["length_us"], off, closed_upto)
+    dt = dict(key=np.uint64, pane_id=np.int64, acc=np.uint64, count=np.uint64, open_seq=np.uint64, max_ts_us=np.int64, closed_upto=np.int64)
+    cols = {n: np.array(v, dtype=dt[n]) for n, v in case["columns"].items()}
     assert len(cols["key"]) > 5
-    snaps = snapshot_rows.window_snapshots(cols, reduction=red, length_us=spec["length_us"], offset_us=off, align_us=ALIGN,
-                                           wait_us=wait * S, now_us=gg.us(gg.NOW), frozen_now_us=gg.us(gg.NOW), classes=win)
-    assert set(snaps) == {str(k) for k in opened_by_key}
-    for ks, lg in logics.items():
-        real = lg.snapshot()
+    snaps = snapshot_rows.window_snapshots(cols, reduction=red, length_us=spec["length_us"], offset_us=off, align_us=spec["align_us"],
+                                           wait_us=wait * S, now_us=now_us, frozen_now_us=now_us)
+    real = case["snapshots"]
+    assert set(snaps) == set(real)
+    for ks, want in real.items():
         mine = snaps[ks]
-        assert list(mine.windower_state.opened) == list(real.windower_state.opened), ks  # same windows, same (first-opened) order
-        assert mine.windower_state == real.windower_state
-        assert {w: (unwrap(v) if red != "count" else v) for w, v in real.logic_states.items()} == mine.logic_states, ks
-        assert (mine.clock_state.watermark_base - mine.clock_state.system_time_of_max_event
-                == real.clock_state.watermark_base - real.clock_state.system_time_of_max_event)
+        # same windows, same (first-opened) order, same bounds
+        assert [[w, _us(m.open_time), _us(m.close_time)] for w, m in mine.windower_state.opened.items()] == want["opened"], ks
+        assert all(not m.merged_ids for m in mine.windower_state.opened.values())
+        assert mine.logic_states == {w: v for w, v in want["logic_states"]}, ks
+        assert _us(mine.clock_state.watermark_base) - _us(mine.clock_state.system_time_of_max_event) == want["clock_delta_us"], ks
+        assert mine.queue == []
     rows = snapshot_rows.recovery_rows("flow.step", snaps, 7)
     assert all(isinstance(pickle.loads(r[3]), win._WindowSnapshot) for r in rows) and [r[1] for r in rows] == sorted(snaps)
     if red == "count":  # (for reduce / max the reference's accumulator is the ITEM; a number resumes count and numeric folds only)
+        builder = _count_builder(spec, now_us)
         resumed = {ks: builder(pickle.loads(pickle.dumps(s))) for ks, s in snaps.items()}
-        got = drive(resumed, builder, batches[cut:], unwrap, cut)
-        got_eof = [(ks, w, tag, unwrap(p) if tag == "E" else None) for ks in sorted(resumed) for w, tag, p in resumed[ks].on_eof()[0] if tag != "M"]
-        assert got == want and got_eof == want_eof
+        got = _drive(resumed, builder, case["batches"][case["cut"]:])
+        got_eof = [[ks, w, tag, p if tag == "E" else None] for ks in sorted(resumed) for w, tag, p in resumed[ks].on_eof()[0] if tag != "M"]
+        assert got == case["want"] and got_eof == case["want_eof"]

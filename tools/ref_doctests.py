@@ -2,9 +2,9 @@
 
 The reference documents every operator with a runnable example and its expected stdout (Sphinx doctest blocks in
 pysrc/bytewax/operators/__init__.py and windowing.py).  This extracts them from the reference tree in place, runs each
-example with `bytewax` aliased to `bytewax_b200`, and compares stdout.  Build container only.
+example with `bytewax` aliased to `bytewax_b200`, and compares stdout.  Needs a reference checkout in $BYTEWAX_SRC.
 
-    python tools/ref_doctests.py            # summary; exit code 1 if any example differs
+    BYTEWAX_SRC=<checkout> python tools/ref_doctests.py            # summary; exit code 1 if any example differs
 """
 import ast
 import contextlib
@@ -14,7 +14,8 @@ import re
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/pysrc/bytewax"
+REF_ROOT = os.environ.get("BYTEWAX_SRC", "")
+REF = os.path.join(REF_ROOT, "pysrc", "bytewax")
 sys.path.insert(0, os.path.join(ROOT, "compat"))
 sys.path.insert(0, ROOT)
 
@@ -54,9 +55,9 @@ def md_examples(path):
 def run_guides(names):
     """(ok, bad) over the guide pages: every page runs in one namespace, cwd = docs/fixtures (pages read sample files)."""
     ok, bad = 0, []
-    docs = "/root/reference/docs/guide"
+    docs = os.path.join(REF_ROOT, "docs", "guide")
     cwd = os.getcwd()
-    os.chdir("/root/reference/docs/fixtures")  # the pages' doctests run beside their fixture files
+    os.chdir(os.path.join(REF_ROOT, "docs", "fixtures"))  # the pages' doctests run beside their fixture files
     try:
         for rel in names:
             ns = {"__name__": "__doctest__"}

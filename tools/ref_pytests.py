@@ -2,9 +2,9 @@
 
 `bytewax` and its submodules are aliased to `bytewax_b200` in `sys.modules`; the reference's `conftest.py`
 (which imports the recovery / tracing modules that are out of scope) is cut off and its two fixtures
-(`entry_point`, `now`) are provided here.  Only usable where /root/reference exists (this container).
+(`entry_point`, `now`) are provided here.  Needs a reference checkout in $BYTEWAX_SRC.
 
-    python tools/ref_pytests.py [pytest args / paths under /root/reference/pytests]
+    BYTEWAX_SRC=<checkout> python tools/ref_pytests.py [pytest args / paths under $BYTEWAX_SRC/pytests]
 """
 import importlib
 import os
@@ -14,7 +14,7 @@ from datetime import datetime, timezone
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/pytests"
+REF = os.path.join(os.environ.get("BYTEWAX_SRC", ""), "pytests")
 sys.path.insert(0, ROOT)
 
 ALIASES = ["", ".dataflow", ".operators", ".operators.windowing", ".operators.helpers", ".testing", ".inputs", ".outputs", ".errors", ".run",
