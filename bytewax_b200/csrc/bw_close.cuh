@@ -304,10 +304,26 @@ __device__ void bw_close_key(const Table& t, const FoldParams& p, const EmitBufs
   }
 }
 
-__global__ void k_close_dirty(Table t, FoldParams p, EmitBufs e, u64 epoch, u32 close_batch) {
+// K4 for the keys on the dirty list.  The last block to finish empties the list and, given the streaming side just
+// folded, its spill list and flags (every block has read the list's length before it counts itself done).
+__global__ void k_close_dirty(Table t, FoldParams p, EmitBufs e, u64 epoch, u32 close_batch, StreamVerdict* sv) {
+  bw_pdl_wait();
+  bw_pdl_launch();
   const u32 n = t.ctr->dirty_count;
   for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
     bw_close_key(t, p, e, t.dirty[i], false, epoch, close_batch);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(&t.ctr->close_done, 1u) == gridDim.x - 1) {
+      t.ctr->close_done = 0;
+      t.ctr->dirty_count = 0;
+      if (sv) {
+        sv->n_spill = 0;
+        sv->flags = 0;
+      }
+    }
+  }
 }
 // EOF: every slot (including the BW_EMPTY_KEY alias slot at index capacity)
 __global__ void k_close_all(Table t, FoldParams p, EmitBufs e, u64 epoch, u32 close_batch) {
@@ -338,4 +354,3 @@ __global__ void k_close_wake(Table t, FoldParams p, EmitBufs e, u64 epoch, u32 c
     bw_close_key(t, p, e, s, false, epoch, close_batch);
   }
 }
-__global__ void k_reset_dirty(Table t) { t.ctr->dirty_count = 0; }

@@ -183,6 +183,17 @@ struct Table {
   struct Counters* ctr;
 };
 
+// verdict of one activation of the streaming path (bw_stream.cuh)
+struct StreamVerdict {
+  u32 clean;   // no row of the activation can be late (prepass rule, bw_prepass.cuh)
+  u32 flags;   // BW_SV_*
+  i64 tmin, tmax;  // event-time span of the activation
+  i64 ts0;     // base of the records' 32-bit relative timestamps (event time of row 0)
+  u32 n_spill; // rows in this activation's spill list
+  u32 pad;
+  i64 gprev;   // running maximum over everything ingested before this activation
+};
+
 struct Counters {
   int free_top;          // free_stack fill
   u32 pool_next;         // bump allocator (node 0 is the null node)
@@ -194,6 +205,8 @@ struct Counters {
   unsigned long long gmax_ts;    // i64 bits: max event ts over everything ingested (prepass chain)
   u32 batch_clean;       // verdict of the prepass for the batch in flight
   u32 n_spill;           // rows in the partial-spill list (bw_stream.cuh)
+  u32 close_done;        // blocks of k_close_dirty that are done (the last one resets; back to 0 after every launch)
+  u32 pad;
 };
 
 // home slot = high part of (scrambled hash) * capacity (no power-of-two constraint on the table).
@@ -340,6 +353,15 @@ __device__ __forceinline__ void bw_reds_min_s64(u32 a, i64 v) { asm volatile("re
 __device__ __forceinline__ void bw_reds_max_s64(u32 a, i64 v) { asm volatile("red.shared.max.s64 [%0], %1;" ::"r"(a), "l"(v) : "memory"); }
 __device__ __forceinline__ void bw_reds_min_u64(u32 a, u64 v) { asm volatile("red.shared.min.u64 [%0], %1;" ::"r"(a), "l"(v) : "memory"); }
 __device__ __forceinline__ void bw_reds_max_u64(u32 a, u64 v) { asm volatile("red.shared.max.u64 [%0], %1;" ::"r"(a), "l"(v) : "memory"); }
+
+// Programmatic dependent launch.  A kernel launched with programmatic stream serialization may start while the
+// kernel before it on the stream is still running; bw_pdl_wait blocks until that kernel has completed and its
+// writes are visible (a no-op for a kernel launched without the attribute).  Every such kernel calls it in every
+// block, before its first access to anything an earlier kernel writes, so that completion stays transitive along
+// the stream.  bw_pdl_launch lets the next kernel's blocks be placed; it hands on nothing (the next kernel waits
+// for this one's completion either way).
+__device__ __forceinline__ void bw_pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void bw_pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 // mbarrier + 1-D bulk async copy (TMA, `cp.async.bulk`): global -> shared, completion counted in
 // bytes on an mbarrier.  SASS: UBLKCP / SYNCS.

@@ -50,15 +50,6 @@ struct __align__(8) SpillRec {  // a row, or a pre-combined partial, for the gen
   u64 weight;  // number of values it stands for
 };
 
-struct StreamVerdict {
-  u32 clean;   // no row of the activation can be late (prepass rule, bw_prepass.cuh)
-  u32 flags;   // BW_SV_*
-  i64 tmin, tmax;  // event-time span of the activation
-  i64 ts0;     // base of the records' 32-bit relative timestamps (event time of row 0)
-  u32 n_spill; // rows in this activation's spill list
-  u32 pad;
-  i64 gprev;   // running maximum over everything ingested before this activation
-};
 // what every rank tells the others about its slice of an activation (multi-GPU verdict: the slices are chained in
 // source-rank order, the arrival order at every destination)
 struct VerdictGather {
@@ -232,11 +223,6 @@ __global__ void __launch_bounds__(BW_SC_THREADS, 1) k_scatter(ScatterArgs A, Fol
   const u32 stg = fbase + (((A.nb * 8 + 15) & ~15u) - A.nb * 4);  // uint4[nb][stg_cap]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const u64 ntiles = (A.n + T - 1) / T;
-  // base of the relative timestamps: event time of row 0
-  i64 ts0 = p.align_us;
-  if (TSM == 0) ts0 = A.ts[0] - p.now_us;
-  else if (TSM == 1) ts0 = p.align_us + (i64)((const u64*)A.vals)[0];
-  if (A.ts0_set) ts0 = A.ts0;
   u32* flags = &A.out.sv->flags;
   u32* n_spill = &A.out.sv->n_spill;
   const u32 seg_mask = (1u << A.seg_shift) - 1u;
@@ -266,6 +252,15 @@ __global__ void __launch_bounds__(BW_SC_THREADS, 1) k_scatter(ScatterArgs A, Fol
   }
   const u32 my_tiles = (ntiles > blockIdx.x) ? (u32)((ntiles - blockIdx.x + gridDim.x - 1) / gridDim.x) : 0u;
   __syncthreads();
+  // Up to here the block has touched only its own shared memory, which overlaps the tail of the kernel before it
+  // on the stream.  From here on it reads the input columns (which the caller may have written with a kernel of
+  // its own on this stream) and writes this side's buckets, counts and verdict fields (read by earlier kernels).
+  bw_pdl_wait();
+  // base of the relative timestamps: event time of row 0
+  i64 ts0 = p.align_us;
+  if (TSM == 0) ts0 = A.ts[0] - p.now_us;
+  else if (TSM == 1) ts0 = p.align_us + (i64)((const u64*)A.vals)[0];
+  if (A.ts0_set) ts0 = A.ts0;
   if (threadIdx.x == 0)
     for (u32 s = 0; s < A.nstage; ++s) {
       const u64 tile = blockIdx.x + (u64)s * gridDim.x;
@@ -652,6 +647,8 @@ k_segfold(SegArgs A, Table t, FoldParams p, EmitBufs e) {
     sink.cap = 512;
     sink.buf = sink_buf;
   }
+  bw_pdl_wait();
+  bw_pdl_launch();
   const u64 ident = (OP <= BW_OP_ADD_F64) ? 0ULL : p.acc_identity;
   const bool tumbling = p.panes_per_offset == 1 && p.panes_per_window == 1;
   for (u32 b = blockIdx.x; b < A.nb; b += gridDim.x) {
@@ -1118,6 +1115,8 @@ __global__ void __launch_bounds__(256) k_spill(Table t, FoldParams p, const Spil
     sink.cap = 256;
     sink.buf = sink_buf;
   }
+  bw_pdl_wait();
+  bw_pdl_launch();
   __syncthreads();
   const u32 n = min(min(sv->n_spill, cap), hi);
   for (u32 i = lo + blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {

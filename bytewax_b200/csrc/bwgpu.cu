@@ -22,6 +22,7 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/bwgpu.h"
@@ -335,6 +336,11 @@ struct bw_fold {
   u32* d_barrier_word = nullptr;
   cudaEvent_t ev_sv[2] = {nullptr, nullptr};
   StreamVerdict* h_sv = nullptr;  // pinned mirror of the two sides' verdicts
+  // One GPU: the verdict runs on a stream of its own, beside the fold stage of the activation before it (nothing on
+  // s_compute reads it; the host does, one activation later).  ev_sv_last: the newest verdict queued there, which
+  // s_compute work that reads or writes Counters::gmax_ts / batch_clean (or copies Counters) waits for.
+  cudaStream_t s_verdict = nullptr;
+  cudaEvent_t ev_scattered = nullptr, ev_sv_last = nullptr;
   // activations with a few late rows (bw_late.cuh); buffers are made on first use
   LateBufs late = {};
   bool late_ready = false;
@@ -813,6 +819,8 @@ static bw_status fold_alloc(bw_fold* f) {
     int prio_lo = 0, prio_hi = 0;
     CU(ctx, cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
     CU(ctx, cudaStreamCreateWithPriority(&f->s_pre, cudaStreamNonBlocking, prio_hi));
+    // the one-block verdict likewise: it runs beside the segment fold and should find room as soon as there is any
+    CU(ctx, cudaStreamCreateWithPriority(&f->s_verdict, cudaStreamNonBlocking, prio_hi));
   }
   if (getenv("BW_NO_OVERLAP")) f->s_x = f->s_compute;  // diagnostic: serialise exchange and fold
   else CU(ctx, cudaStreamCreateWithFlags(&f->s_x, cudaStreamNonBlocking));
@@ -822,6 +830,7 @@ static bw_status fold_alloc(bw_fold* f) {
   CU(ctx, cudaEventCreateWithFlags(&f->ev_in, cudaEventDisableTiming));
   CU(ctx, cudaEventCreateWithFlags(&f->ev_pre, cudaEventDisableTiming));
   CU(ctx, cudaEventCreateWithFlags(&f->ev_h2d, cudaEventDisableTiming));
+  CU(ctx, cudaEventCreateWithFlags(&f->ev_scattered, cudaEventDisableTiming));
   // No persisting-L2 carve-out: measured on this part (profiles/r01_notes.md) a 64 MiB persisting
   // window on the hot slots leaves too little normal L2 for the second-pane array and slows
   // window-boundary activations by 15-30 %; plain LRU + evict_first input loads is faster.
@@ -1069,6 +1078,8 @@ void bw_fold_destroy(bw_fold* f) {
   if (f->s_compute) cudaStreamDestroy(f->s_compute);
   if (f->s_copy) cudaStreamDestroy(f->s_copy);
   if (f->s_pre) cudaStreamDestroy(f->s_pre);
+  if (f->s_verdict) cudaStreamDestroy(f->s_verdict);
+  if (f->ev_scattered) cudaEventDestroy(f->ev_scattered);
   if (f->s_x && f->s_x != f->s_compute) cudaStreamDestroy(f->s_x);
   if (f->ev_in) cudaEventDestroy(f->ev_in);
   if (f->ev_gen) cudaEventDestroy(f->ev_gen);
@@ -1234,14 +1245,35 @@ static bw_status exchange(bw_fold* f, const u64* d_keys, const void* d_vals, con
   return BW_OK;
 }
 
-// K4 for the keys the fold marked, then the end-of-activation resets
+// A kernel that may be placed while the kernel before it on the stream is still running (programmatic dependent
+// launch): its launch and its prologue overlap the other's tail.  It must call bw_pdl_wait (bw_common.cuh) in every block.
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t s, Args&&... args) {
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)grid);
+  cfg.blockDim = dim3((unsigned)block);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = s;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
+
+// Work queued on `s` after this sees every verdict queued so far (one GPU: they run on s_verdict).
+static bw_status verdict_join(bw_fold* f, cudaStream_t s) {
+  if (f->ev_sv_last) CU(f->ctx, cudaStreamWaitEvent(s, f->ev_sv_last, 0));
+  return BW_OK;
+}
+
+// K4 for the keys the fold marked; its last block does the end-of-activation resets
 static bw_status close_stage(bw_fold* f, u64 ord, u32 batch_no, StreamVerdict* sv) {
   bw_ctx* ctx = f->ctx;
   f->pt.mark(4, 0, f->s_compute);
-  k_close_dirty<<<f->close_grid, 256, 0, f->s_compute>>>(f->t, f->p, f->e, ord, batch_no);
-  k_stream_reset<<<1, 1, 0, f->s_compute>>>(f->t, sv);
-  CU(ctx, cudaGetLastError());
-  f->st.kernel_launches += 2;
+  CU(ctx, launch_pdl(k_close_dirty, f->close_grid, 256, 0, f->s_compute, f->t, f->p, f->e, ord, batch_no, sv));
+  f->st.kernel_launches++;
   f->pt.mark(4, 1, f->s_compute);
   return BW_OK;
 }
@@ -1288,9 +1320,8 @@ static bw_status direct_fold(bw_fold* f, const BatchView& bv, u64 known, u32 bat
       f->pt.ev[3][1].push_back(ep->b);
     }
     if (i + 1 < n_sub) {
-      k_close_dirty<<<f->close_grid, 256, 0, f->s_compute>>>(f->t, f->p, f->e, ord, batch_no);
-      k_reset_dirty<<<1, 1, 0, f->s_compute>>>(f->t);
-      f->st.kernel_launches += 2;
+      k_close_dirty<<<f->close_grid, 256, 0, f->s_compute>>>(f->t, f->p, f->e, ord, batch_no, nullptr);
+      f->st.kernel_launches++;
     }
   }
   return BW_OK;
@@ -1356,25 +1387,34 @@ static bw_status stream_front(bw_fold* f, const u64* d_keys, const void* d_vals,
     CU(ctx, cudaEventRecord(ep->a, s));
   }
   f->pt.mark(5, 0, s);
-  if (grid) f->scatter_kernel<<<grid, BW_SC_THREADS, f->scatter_smem, s>>>(A, f->p);
+  if (grid) CU(ctx, launch_pdl(f->scatter_kernel, grid, BW_SC_THREADS, f->scatter_smem, s, A, f->p));
   if (ep) CU(ctx, cudaEventRecord(ep->b, s));  // (the scatter kernel alone: the one-block verdict is timed apart)
+  // One GPU: the verdict goes to its own stream once the scatter is done, and s_compute goes straight on to the fold
+  // stage of the activation before.  Multi-GPU: it stays on s_compute (the gather behind it is a collective there).
+  cudaStream_t vs = s;
+  if (!multi) {
+    vs = f->s_verdict;
+    CU(ctx, cudaEventRecord(f->ev_scattered, s));
+    CU(ctx, cudaStreamWaitEvent(vs, f->ev_scattered, 0));
+  }
   EventPair* ev = next_timer(f, batch_no);
   if (ev) {
     ev->rows = 0;
     ev->kind = 2;
-    CU(ctx, cudaEventRecord(ev->a, s));
+    CU(ctx, cudaEventRecord(ev->a, vs));
   }
-  if (f->p.ts_from_value == 2) k_verdict_none<<<1, 1, 0, s>>>(f->p, f->d_ctr, sb.side[side].sv, vg, rows);
+  if (f->p.ts_from_value == 2) k_verdict_none<<<1, 1, 0, vs>>>(f->p, f->d_ctr, sb.side[side].sv, vg, rows);
   else
-    k_verdict<<<1, 1024, 0, s>>>(A.tile_min, A.tile_max, A.tile_bad, (u32)ntiles, f->p, f->d_ctr, sb.side[side].sv,
-                                 f->has_ts ? d_ts : nullptr, (const u64*)d_vals, vg);
+    k_verdict<<<1, 1024, 0, vs>>>(A.tile_min, A.tile_max, A.tile_bad, (u32)ntiles, f->p, f->d_ctr, sb.side[side].sv,
+                                  f->has_ts ? d_ts : nullptr, (const u64*)d_vals, vg);
   CU(ctx, cudaGetLastError());
-  f->pt.mark(5, 1, s);
-  if (ev) CU(ctx, cudaEventRecord(ev->b, s));
+  f->pt.mark(5, 1, vs);
+  if (ev) CU(ctx, cudaEventRecord(ev->b, vs));
   f->st.kernel_launches += 2;
-  CU(ctx, cudaMemcpyAsync(&f->h_sv[side], sb.side[side].sv, sizeof(StreamVerdict), cudaMemcpyDeviceToHost, s));
+  CU(ctx, cudaMemcpyAsync(&f->h_sv[side], sb.side[side].sv, sizeof(StreamVerdict), cudaMemcpyDeviceToHost, vs));
   if (multi) f->vg_pending[side] = true;  // gathered by the next collective on the stream (gather_verdict)
-  CU(ctx, cudaEventRecord(f->ev_sv[side], s));
+  CU(ctx, cudaEventRecord(f->ev_sv[side], vs));
+  if (!multi) f->ev_sv_last = f->ev_sv[side];
   return BW_OK;
 }
 
@@ -1407,6 +1447,10 @@ static bw_status legacy_batch(bw_fold* f, const u64* d_keys, const void* d_vals,
   bool clean = true;
   if (f->p.track_wm && max_total > 0) {
     if (pre_stream != f->s_compute && ctx->world == 1 && f->pre_wait) CU(ctx, cudaStreamWaitEvent(pre_stream, f->pre_wait, 0));
+    {  // (k_prepass_scan chains from Counters::gmax_ts)
+      bw_status vst = verdict_join(f, pre_stream);
+      if (vst != BW_OK) return vst;
+    }
     const u64 nranges = (max_total + BW_RANGE_ROWS - 1) / BW_RANGE_ROWS;
     // one warp per 2048-row range; cap at 64 warps per SM in total (the block size is small so that a block fits beside the fold)
     int grid = (int)std::min<u64>((nranges * 32 + BW_PRE_THREADS - 1) / BW_PRE_THREADS, (u64)ctx->sm_count * (2048 / BW_PRE_THREADS));
@@ -1619,6 +1663,10 @@ static bw_status late_split(bw_fold* f, const Deferred& d, const BatchView& bv, 
   const StreamBufs& sb = f->sb;
   cudaStream_t s = f->s_compute;
   *ok = false;
+  {
+    bw_status vst = verdict_join(f, s);
+    if (vst != BW_OK) return vst;
+  }
   LateBufs& L = f->late;
   if (!f->late_ready) {
     const u64 maxr = f->spec.max_batch_rows;
@@ -1759,12 +1807,14 @@ static bw_status stream_resolve(bw_fold* f) {
     }
     f->pt.mark(6, 0, s);
     const int grid = (int)std::min<u32>(sb.nb, (u32)f->segfold_grid);
-    f->segfold_kernel<<<grid, BW_SF_THREADS, f->segfold_smem, s>>>(A, f->t, f->p, f->e);
-    CU(ctx, cudaGetLastError());
+    CU(ctx, launch_pdl(f->segfold_kernel, grid, BW_SF_THREADS, f->segfold_smem, s, A, f->t, f->p, f->e));
     f->pt.mark(6, 1, s);
     if (ep) CU(ctx, cudaEventRecord(ep->b, s));
     f->pt.mark(7, 0, s);
-    k_spill<<<ctx->sm_count, 256, 0, s>>>(f->t, f->p, sb.side[d.side].spill, sb.side[d.side].sv, sb.spill_cap, d.batch_no, n_pre, 0xFFFFFFFFu);
+    // (what the segment fold set aside; nearly always nothing, and only the device knows: the launch overlaps the
+    // fold's tail and the kernel finds the list empty)
+    CU(ctx, launch_pdl(k_spill, ctx->sm_count, 256, 0, s, f->t, f->p, (const SpillRec*)sb.side[d.side].spill,
+                       (const StreamVerdict*)sb.side[d.side].sv, sb.spill_cap, d.batch_no, n_pre, 0xFFFFFFFFu));
     f->st.kernel_launches += 2;
     f->st.fold_launches++;
     f->st.combined_folds++;
@@ -1772,6 +1822,10 @@ static bw_status stream_resolve(bw_fold* f) {
     f->pt.mark(7, 1, s);
   } else {
     // (the scatter output of this activation is simply not read)
+    {  // the direct and sort paths' kernels see the verdict chain as it stood on s_compute before
+      bw_status vst = verdict_join(f, s);
+      if (vst != BW_OK) return vst;
+    }
     if (split) sv = f->h_sv[d.side], sv.clean = 0u;  // (split, but too many panes for the segment fold: the sort path; nothing was emitted)
     if (sv.clean) {
       st = direct_fold(f, bv, d.rows, d.batch_no, d.ord, sv.tmin, sv.tmax);
@@ -2158,6 +2212,10 @@ static bw_status flush_rows(bw_fold* f) {
 static bw_status collect(bw_fold* f, bw_emit* out) {
   bw_ctx* ctx = f->ctx;
   cudaStream_t s = f->s_compute;
+  {
+    bw_status vst = verdict_join(f, s);
+    if (vst != BW_OK) return vst;
+  }
   CU(ctx, cudaMemcpyAsync(f->h_ctr, f->d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
   CU(ctx, cudaStreamSynchronize(s));
   if (f->s_out) CU(ctx, cudaStreamSynchronize(f->s_out));
@@ -2271,6 +2329,10 @@ bw_status bw_snapshot_take(bw_fold* f, bw_snapshot* out) {
   }
   cudaStream_t s = f->s_compute;
   if (f->s_x) CU(ctx, cudaStreamSynchronize(f->s_x));
+  {
+    bw_status vst = verdict_join(f, s);
+    if (vst != BW_OK) return vst;
+  }
   if (!f->d_snap_ctr) CU(ctx, dmalloc(&f->d_snap_ctr, 2));
   CU(ctx, cudaMemsetAsync(f->d_snap_ctr, 0, 2 * sizeof(unsigned long long), s));
   k_snap_count<<<f->close_grid, 256, 0, s>>>(f->t, f->d_snap_ctr);
@@ -2327,11 +2389,14 @@ bw_status bw_snapshot_load(bw_fold* f, const bw_snapshot* in) {
     k_snap_load<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(f->t, f->p, dc, n, (u32)in->batch_no, ctx->world, ctx->rank);
     CU(ctx, cudaGetLastError());
     // re-rank every restored key (newest pane into the hot slot); nothing is closable in a state dumped after an advance
-    k_close_dirty<<<f->close_grid, 256, 0, s>>>(f->t, f->p, f->e, in->last_epoch, (u32)in->batch_no);
-    k_reset_dirty<<<1, 1, 0, s>>>(f->t);
-    f->st.kernel_launches += 3;
+    k_close_dirty<<<f->close_grid, 256, 0, s>>>(f->t, f->p, f->e, in->last_epoch, (u32)in->batch_no, nullptr);
+    f->st.kernel_launches += 2;
     CU(ctx, cudaStreamSynchronize(s));
     cudaFree(dev);
+  }
+  {
+    bw_status vst = verdict_join(f, s);
+    if (vst != BW_OK) return vst;
   }
   k_snap_set_gmax<<<1, 1, 0, s>>>(f->d_ctr, (i64)in->gmax_ts_us);
   CU(ctx, cudaMemcpyAsync(f->h_ctr, f->d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
@@ -2377,6 +2442,7 @@ bw_status bw_fold_stats(bw_fold* f, bw_stats* out) {
     bw_status st = stream_resolve(f);
     if (st != BW_OK) return st;
   }
+  CU(f->ctx, cudaStreamSynchronize(f->s_verdict));
   CU(f->ctx, cudaStreamSynchronize(f->s_compute));
   drain_timers(f);
   *out = f->st;
@@ -2388,6 +2454,7 @@ bw_status bw_fold_reset_timers(bw_fold* f) {
     bw_status st = stream_resolve(f);
     if (st != BW_OK) return st;
   }
+  CU(f->ctx, cudaStreamSynchronize(f->s_verdict));
   CU(f->ctx, cudaStreamSynchronize(f->s_compute));
   drain_timers(f);
   f->st.sum_scatter_ms = 0;
@@ -2412,6 +2479,7 @@ bw_status bw_fold_sync(bw_fold* f) {
   CU(f->ctx, cudaStreamSynchronize(f->s_copy));
   CU(f->ctx, cudaStreamSynchronize(f->s_pre));
   CU(f->ctx, cudaStreamSynchronize(f->s_x));
+  CU(f->ctx, cudaStreamSynchronize(f->s_verdict));
   CU(f->ctx, cudaStreamSynchronize(f->s_compute));
   return BW_OK;
 }
@@ -2431,6 +2499,7 @@ bw_status bw_fold_time_begin(bw_fold* f) {
   CU(ctx, cudaStreamSynchronize(f->s_copy));
   CU(ctx, cudaStreamSynchronize(f->s_pre));
   CU(ctx, cudaStreamSynchronize(f->s_x));
+  CU(ctx, cudaStreamSynchronize(f->s_verdict));
   CU(ctx, cudaStreamSynchronize(f->s_compute));
   CU(ctx, cudaEventRecord(f->ev_t0, f->s_compute));
   return BW_OK;
@@ -2445,6 +2514,10 @@ bw_status bw_fold_time_end(bw_fold* f, float* ms) {
   CU(ctx, cudaStreamSynchronize(f->s_copy));
   CU(ctx, cudaStreamSynchronize(f->s_pre));
   CU(ctx, cudaStreamSynchronize(f->s_x));
+  {  // (every verdict is done by now: stream_resolve has waited for the newest; the stop event is behind them anyway)
+    bw_status vst = verdict_join(f, f->s_compute);
+    if (vst != BW_OK) return vst;
+  }
   CU(ctx, cudaEventRecord(f->ev_t1, f->s_compute));
   CU(ctx, cudaEventSynchronize(f->ev_t1));
   CU(ctx, cudaEventElapsedTime(ms, f->ev_t0, f->ev_t1));
